@@ -5,14 +5,21 @@ SparkAffineFusion's config (64 tiles -> 2048^3 float32) as the `fusion` sub-obje
 
     python bench.py --gpus N --steps K --warmup W          (N>1: launched under torchrun)
     python bench.py --impl reference ...                    (CPU arm: the oracle port on host cores)
+    python bench.py ... --dump-outputs DIR                  (also write rank 0's outputs as DIR/<name>.npy)
 
 A "step" is one pass of the hot path over the whole batch (112 pairs).  `value` is measured
 with the crops resident in HBM; `e2e` goes through the same C-ABI call with pinned HOST
-buffers (H2D inside the timed region).  One JSON line is printed by rank 0.
+buffers (H2D inside the timed region).  Every timed section runs K steps.  One JSON line is
+printed by rank 0.
+
+--dump-outputs writes what the last timed step of each GPU section returned: the phase-correlation
+results (pcm_*, pcm_e2e_*), a fixed seeded sample of the fused volume (fusion_sample*) and the DoG
+detections (dog_*).  All inputs are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
+import dataclasses
 import json
 import multiprocessing as mp
 import os
@@ -28,6 +35,7 @@ sys.path.insert(0, ROOT)
 
 METRIC = "tile-pairs/sec (phase-corr, 512^3 uint16 overlaps)"
 UNIT = "pairs/s"
+DUMP_SAMPLE = 1 << 21      # voxels of the fused volume that --dump-outputs keeps (24 MB with their indices)
 
 
 # ------------------------------------------------------------------------------------------ utils
@@ -99,6 +107,21 @@ def ncu_traffic(tag):
         return int(json.load(open(p))["bytes_per_launch"][tag])
     except Exception:
         return None
+
+
+def dump(dirname, name, values):
+    """--dump-outputs: one output array as ``dirname/name.npy``; float32 stays float32, everything else becomes float64."""
+    if dirname is None:
+        return
+    os.makedirs(dirname, exist_ok=True)
+    a = np.asarray(values)
+    np.save(os.path.join(dirname, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
+def dump_pcm(dirname, prefix, results):
+    """one array per PcmResult field, one row per pair"""
+    for f in dataclasses.fields(results[0]):
+        dump(dirname, f"{prefix}_{f.name}", [getattr(r, f.name) for r in results])
 
 
 def pcm_bytes_per_pair(n, P, K_px):
@@ -377,8 +400,8 @@ def run_gpu(args, rank, world, local_rank):
 
     def timed(fn, steps):
         """K steps between barrier + synchronize on both sides, device time by CUDA events on the launching stream, max
-        over ranks.  A step that raises still completes this call's collectives (then re-raises), so the other ranks
-        are never left alone inside a barrier."""
+        over ranks; ``timed.last`` is what the last step returned.  A step that raises still completes this call's
+        collectives (then re-raises), so the other ranks are never left alone inside a barrier."""
         timed_calls[0] += 1
         barrier()
         e0 = torch.cuda.Event(enable_timing=True)
@@ -388,7 +411,7 @@ def run_gpu(args, rank, world, local_rank):
         err = None
         try:
             for _ in range(steps):
-                fn()
+                timed.last = fn()
         except Exception as exc:
             err = exc
         e1.record(stream)
@@ -458,6 +481,7 @@ def run_gpu(args, rank, world, local_rank):
     ms, wall_ms = timed(step_resident, args.steps)
     launches = ctx.launch_count() - l0
     clocks = sampler.stop()
+    dump_pcm(args.dump_outputs, "pcm", timed.last)
     ms_per_step = ms / args.steps
     value = world * npairs / (ms_per_step / 1000.0)
 
@@ -511,6 +535,7 @@ def run_gpu(args, rank, world, local_rank):
             good += int(r.found and tuple(r.shift_int) == want)
         step_host()
         e2e_ms, _ = timed(step_host, args.steps)
+        dump_pcm(args.dump_outputs, "pcm_e2e", timed.last)
         e2e_value = world * len(gpairs) / (e2e_ms / args.steps / 1000.0)
         return {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": len(used) * n ** 3 * 2,
                "d2h_bytes_per_step": len(gpairs) * 2400, "ms_per_step": e2e_ms / args.steps,
@@ -622,8 +647,11 @@ def bench_dog(args, ctx, stream, dev, rank, world, timed, peak_gbs):
             found.extend(ctx.dog_detect(h, lo, sz, sigma=1.8, threshold=0.008, min_intensity=0.0, max_intensity=4000.0))
     step()
     nfound = len({p[2] for p in found})
-    ms, _ = timed(step, max(1, min(args.steps, 2)))
-    ms /= max(1, min(args.steps, 2))
+    ms, _ = timed(step, args.steps)
+    ms /= args.steps
+    if args.dump_outputs:
+        for i, name in enumerate(("loc", "value", "voxel", "is_max")):
+            dump(args.dump_outputs, "dog_" + name, [p[i] for p in found])
     nvox = n * n * nz
     ctx.volume_free(h)
     return {"metric": "DoG interest points, Mvoxels/sec", "value": world * nvox / (ms / 1000.0) / 1e6, "unit": "Mvoxels/s", "ms_per_step": ms,
@@ -697,6 +725,10 @@ def bench_fusion(args, ctx, stream, dev, rank, world, timed, peak_gbs, peak_src)
     ms_step, launches, step_resident = run_variant("AVG_BLEND", vd, args.steps)
     launches //= args.steps
     value = nvox_total / (ms_step / 1000.0) / 1e6
+    if args.dump_outputs:   # before the variants below overwrite `out`
+        idx = np.sort(np.random.default_rng(0).choice(nvox_rank, min(DUMP_SAMPLE, nvox_rank), replace=False))
+        dump(args.dump_outputs, "fusion_sample_index", idx)
+        dump(args.dump_outputs, "fusion_sample", out[torch.from_numpy(idx).to(dev)].cpu().numpy())
 
     # ---- parity spot check against the C oracle, outside the timed region: one super-block at a 8-tile junction
     oracle_check = None
@@ -752,7 +784,7 @@ def bench_fusion(args, ctx, stream, dev, rank, world, timed, peak_gbs, peak_src)
         models_rot = m2
         vd_rot = {v: dict(src_to_world=models_rot[v], vol_handle=handles[v], blend_border=bf.adjust_blending(models_rot[v])[0],
                           blend_range=bf.adjust_blending(models_rot[v])[1]) for v in mine}
-        ms_r, _, _ = run_variant("AVG_BLEND", vd_rot, max(1, min(args.steps, 2)))
+        ms_r, _, _ = run_variant("AVG_BLEND", vd_rot, args.steps)
         variants["rotated_0.5deg_z"] = {"value": nvox_total / (ms_r / 1000.0) / 1e6, "unit": "Mvoxels/s", "ms_per_step": ms_r,
                                         "kernel": "fuse_tma_kernel<general> (xy-affine z-marching tiles for <= 2 views, per-voxel tiles otherwise)"}
         # a rotation about an oblique axis has no exploitable structure: every voxel samples 8 taps
@@ -767,7 +799,7 @@ def bench_fusion(args, ctx, stream, dev, rank, world, timed, peak_gbs, peak_src)
             models_obl.append(np.hstack([Rg, (t + c - Rg @ c)[:, None]]))
         vd_obl = {v: dict(src_to_world=models_obl[v], vol_handle=handles[v], blend_border=bf.adjust_blending(models_obl[v])[0],
                           blend_range=bf.adjust_blending(models_obl[v])[1]) for v in mine}
-        ms_o, _, _ = run_variant("AVG_BLEND", vd_obl, 1)
+        ms_o, _, _ = run_variant("AVG_BLEND", vd_obl, args.steps)
         variants["rotated_0.5deg_oblique"] = {"value": nvox_total / (ms_o / 1000.0) / 1e6, "unit": "Mvoxels/s", "ms_per_step": ms_o,
                                               "kernel": "fuse_tma_kernel<general> (per-voxel 8-tap tiles)"}
         if not args.skip_fusion_content:
@@ -781,7 +813,7 @@ def bench_fusion(args, ctx, stream, dev, rank, world, timed, peak_gbs, peak_src)
             ctx.synchronize()
             pre_s = time.perf_counter() - t0
             vd_c = {v: dict(vd[v], content_handle=chandle[tiles[v].data_ptr()]) for v in mine}
-            ms_c, _, _ = run_variant("AVG_BLEND_CONTENT", vd_c, 1)
+            ms_c, _, _ = run_variant("AVG_BLEND_CONTENT", vd_c, args.steps)
             variants["content_based"] = {"value": nvox_total / (ms_c / 1000.0) / 1e6, "unit": "Mvoxels/s", "ms_per_step": ms_c,
                                          "fusion_type": "AVG_BLEND_CONTENT", "sigma": [20.0, 40.0],
                                          "alg_bytes_per_voxel": 12.54, "kernel": "fuse_tma_kernel<translation, content> (content taps from global memory)",
@@ -848,7 +880,7 @@ def bench_fusion(args, ctx, stream, dev, rank, world, timed, peak_gbs, peak_src)
                         ctx.volume_free(h)
             return step_host
 
-        nst = max(1, min(args.steps, 2))
+        nst = args.steps
         ring_f32 = torch.empty((ring_n, 256 * 256 * 128), dtype=torch.float32).pin_memory()
         step_host = make_step(nat.DTYPE_F32, ring_f32)
         step_host()
@@ -921,9 +953,8 @@ def bench_fusion(args, ctx, stream, dev, rank, world, timed, peak_gbs, peak_src)
                 ctx.fuse_finish(swi, sw, nb, pvs, outd)
             for _ in range(3):
                 step_vs()
-            reps = 10
-            ms_vs, _ = timed(step_vs, reps)
-            ms_vs /= reps
+            ms_vs, _ = timed(step_vs, args.steps)
+            ms_vs /= args.steps
             view_sharded = {"value": nb / (ms_vs / 1000.0) / 1e6, "unit": "Mvoxels/s", "ms_per_block": ms_vs,
                             "block": list(bsz), "views_total": len(vids), "views_on_rank0": len(my),
                             "allreduce_bytes_per_block": 2 * nb * 4,
@@ -972,10 +1003,15 @@ def main():
     ap.add_argument("--fusion-stride", type=int, default=491)
     ap.add_argument("--fusion-size", type=int, default=2048)
     ap.add_argument("--fusion-distinct", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's outputs of the last timed steps as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if rank != 0:
+        args.dump_outputs = None
     wd = int(os.environ.get("BS_BENCH_WATCHDOG", "0"))
     if wd > 0:      # debugging aid for multi-rank runs: every `wd` seconds each rank dumps where it is
         import faulthandler
